@@ -1,6 +1,6 @@
 """bench.py -- Monte-Carlo free-integration throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     torchrun ... bench.py --gpus N ...          (one rank per GPU, NCCL)
 
 Workload = BASELINE.json configs[1]: free_integration on motion_def-90deg_turn.csv
@@ -18,6 +18,11 @@ history (72 B per run-step) to the host, which is what the reference's Sim.run l
 L2 is flushed between timed steps.  `extra` carries the other BASELINE configurations measured in
 the same process (config 3 sharded over the ranks, config 4 at N = 1) and, for N > 1, the check
 that the sharded statistics equal the single-GPU ones.  See DESIGN.md section 7.
+
+--steps K sets the number of steps of every timed loop.  --dump-outputs DIR writes what the last
+timed step returned as float64 .npy files: end_err.npy (per-run end-point errors of rank 0's runs,
+[1000, 9]) and error_stats.npy (ensemble max|e| / mean / std, [3, 9]).  The inputs are fixed (frozen
+trajectory, fixed seed), so two builds can be compared output for output.
 """
 import argparse
 import ctypes
@@ -34,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it
 _REAL_STDOUT = None
 
 
@@ -278,6 +284,13 @@ def cpu_baseline_sample(g, nav, imu, budget_s=4.0):
 
 
 # ------------------------------------------------------------------ B200 arm ---------------------
+def dump_outputs(path, arrays):
+    """--dump-outputs: one float64 .npy per array the timed step returned."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def roofline_inputs(lanes, shape):
     """FP64 instructions per run-step and DRAM bytes per launch of the dominant kernel, from the
     committed ncu summary named in profiles/roofline_inputs_r02.json -- valid only for the launch
@@ -375,6 +388,8 @@ def run_b200(args):
     dev_ms = allmax(sum(a.elapsed_time(b) for a, b in evs))
     value = total_runs * n * args.steps / (dev_ms * 1e-3)
     stats = stats.cpu().numpy().copy() if hasattr(stats, 'cpu') else stats
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'end_err': res.end_err.cpu().numpy(), 'error_stats': stats})
     k3x_timed_out = bool(p2p.timed_out()) if p2p is not None else False
 
     # ---- N > 1: the sharded statistics against ONE GPU doing all the runs -------------------
@@ -390,7 +405,7 @@ def run_b200(args):
 
     # ---- dominant kernel alone: launch duration -> roofline --------------------------------
     kev = []
-    for _ in range(max(args.steps, 5)):
+    for _ in range(args.steps):
         flush.fill_(1)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
@@ -469,7 +484,7 @@ def run_b200(args):
         return total_runs * n * steps / allmax(time.perf_counter() - t0)
 
     e2e_value = timed_e2e(False, args.steps)
-    e2e_hist_value = timed_e2e(True, max(3, args.steps // 2))
+    e2e_hist_value = timed_e2e(True, args.steps)
     # plan path (N = 1): true IMU samples + last ref_nav row + initial state up,
     # statistics + per-run end-point errors down
     h2d = (n * 6 + 9 + 9) * 8
@@ -697,7 +712,11 @@ def main():
     ap.add_argument('--c3-runs', type=int, default=C3_RUNS, help='Monte-Carlo runs of the config-3 block')
     ap.add_argument('--no-config4', action='store_true')
     ap.add_argument('--c5-runs', type=int, default=10000, help='Monte-Carlo runs of the config-5 block')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the last timed step\'s end-point errors and statistics to DIR/*.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

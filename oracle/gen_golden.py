@@ -491,10 +491,12 @@ def gen_pathgen():
 
 
 def gen_allan():
-    rng = np.random.RandomState(2024)
+    seed = 2024
+    rng = np.random.RandomState(seed)
     fs = 100.0
     n = 180000
     # white + random walk + a GM-like component: exercises all tau decades
+    # (tests/conftest.py:allan_golden regenerates x from the seed: the series alone is 1.4 MB)
     x = 0.01 * rng.randn(n) + np.cumsum(1e-5 * rng.randn(n))
     avar, tau = allan.allan_var(x, fs)
     x2 = rng.randn(7351)       # ragged: n not a multiple of anything
@@ -502,8 +504,8 @@ def gen_allan():
     x3 = rng.randn(800)        # too short: max_bin*ts < 1 -> ([], [])
     a3, t3 = allan.allan_var(x3, 100.0)
     assert len(a3) == 0
-    np.savez_compressed(os.path.join(OUT, 'allan.npz'), fs=fs, x=x, avar=avar, tau=tau,
-                        fs2=50.0, x2=x2, avar2=avar2, tau2=tau2, x3=x3)
+    np.savez_compressed(os.path.join(OUT, 'allan.npz'), fs=fs, seed=seed, n=n, x_every_1000=x[::1000],
+                        avar=avar, tau=tau, fs2=50.0, x2=x2, avar2=avar2, tau2=tau2, x3=x3)
 
 
 def gen_allan_config4(n=14400000, fs=400.0, seed=5, run=2):

@@ -19,6 +19,18 @@ def load_golden(name):
     return dict(np.load(os.path.join(GOLDEN, name), allow_pickle=False))
 
 
+def allan_golden():
+    """allan.npz with its 180 000-sample series `x` regenerated from the stored seed, as
+    oracle/gen_golden.py made it (NumPy's RandomState stream is frozen); every 1000th stored
+    sample pins the regeneration."""
+    g = load_golden('allan.npz')
+    n = int(g['n'])
+    rng = np.random.RandomState(int(g['seed']))
+    g['x'] = 0.01 * rng.randn(n) + np.cumsum(1e-5 * rng.randn(n))
+    assert np.array_equal(g['x'][::1000], g['x_every_1000']), 'allan.npz: regenerated series differs'
+    return g
+
+
 @pytest.fixture(scope='session')
 def golden():
     return load_golden

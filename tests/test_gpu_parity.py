@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import oracle_np as onp
-from conftest import load_golden, assert_close, wrap_pi
+from conftest import allan_golden, load_golden, assert_close, wrap_pi
 
 pytestmark = pytest.mark.gpu
 
@@ -255,7 +255,7 @@ def test_k3_stats_vs_numpy(eng):
 
 
 def test_k4_allan_vs_reference(eng):
-    g = load_golden('allan.npz')
+    g = allan_golden()
     x = _dev(g['x'])
     avar, tau = eng.allan(float(g['fs']), x, x.numel(), 1)
     assert_close(tau.cpu().numpy(), g['tau'], 1e-15, 0.0, 'tau')
@@ -329,8 +329,8 @@ def test_host_entry_points(eng):
                                                       hp(ini), hp(end_err), hp(stats)))
     gs = np.concatenate([g['stat_att_euler_std'], g['stat_pos_std'], g['stat_vel_std']])
     assert_close(stats[2], gs, 1e-6, 1e-3, 'std')
-    x = np.ascontiguousarray(load_golden('allan.npz')['x'])
-    ga = load_golden('allan.npz')
+    ga = allan_golden()
+    x = np.ascontiguousarray(ga['x'])
     avar, tau = np.empty(38), np.empty(38)
     _lib.check(lib.b2ins_allan_f64_host(100.0, x.size, 1, hp(x), 1, x.size, 1, hp(avar), hp(tau)))
     assert_close(avar, ga['avar'], 1e-9, 0.0, 'avar')

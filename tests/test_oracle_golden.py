@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 import oracle_np as onp
-from conftest import load_golden, assert_close, wrap_pi
+from conftest import allan_golden, load_golden, assert_close, wrap_pi
 
 TIGHT = 1e-12
 
@@ -90,7 +90,7 @@ def test_normals_are_standard():
 
 
 def test_allan_matches_reference():
-    g = load_golden('allan.npz')
+    g = allan_golden()
     avar, tau = onp.allan_var(g['x'], float(g['fs']))
     assert_close(tau, g['tau'], 1e-15, what='tau')
     assert_close(avar, g['avar'], 1e-12, 0.0, what='avar')
